@@ -49,6 +49,35 @@ def synth_batch(B, T, L, seed):
     return x, targets, pct, tsz
 
 
+DUMP_MAX_ELEMS = 1 << 17
+
+
+def dump_outputs(path, loss, state, grads):
+    """--dump-outputs: what the last timed step hands its caller, as <path>/<name>.npy: `loss`, the model's state_dict
+    after the optimizer step (parameters and BatchNorm running statistics, under their state_dict keys) and every
+    parameter's gradient of that step (`grad.<key>`).  float32, integer buffers as float64.  A tensor of more than
+    DUMP_MAX_ELEMS elements is stored as that many values at fixed positions (numpy default_rng(0), sorted flat
+    indices), which keeps the largest workload (stress) below 64 MB in all.  At the default precision the librispeech
+    step sums its gradients in a fixed order: two runs with the same arguments write identical values.  Other
+    workloads and --precision fp32 can reach kernels that still add with float atomics (the lookahead weight
+    gradient, the FFMA conv weight / bias gradients, column sums where the recurrent sweep does not produce the bias
+    gradients), so their dumps may differ in the last bits from run to run.  The conv biases feed BatchNorm: their
+    true gradient is zero and what is dumped for them is rounding noise, not meaningful across builds."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {"loss": np.array([loss], np.float64)}
+    for prefix, tensors in (("", state), ("grad.", grads)):
+        for k, v in tensors.items():
+            a = v.detach().cpu().numpy()
+            a = a.astype(np.float32 if v.is_floating_point() else np.float64)
+            if a.size > DUMP_MAX_ELEMS:
+                a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+            arrays[prefix + k] = a
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log(f"dumped {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 2**20:.1f} MiB) to {path}")
+
+
 def log(msg):
     if int(os.environ.get("RANK", "0")) == 0:
         print(f"[bench +{time.time() - T0:6.1f}s] {msg}", file=sys.stderr, flush=True)
@@ -466,9 +495,15 @@ def run_b200(args):
         sampler.start()
     ms_dev, launches, loss_val = timed(args.steps, e2e=False)
     log(f"device-resident: {ms_dev:.2f} ms/step")
+    if args.dump_outputs and rank == 0:      # device copies now, written out once the timed windows are over
+        dump = (loss_val, {k: v.detach().clone() for k, v in model.state_dict().items()},
+                {k: p.grad.detach().clone() for k, p in model.named_parameters()})
     ms_e2e, _, _ = timed(args.steps, e2e=True)
     log(f"e2e: {ms_e2e:.2f} ms/step")
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *dump)
+        del dump
 
     # ---- per-block device times (cudaEvent ranges inside the library) for the roofline of the dominant kernel
     prof = {}
@@ -603,7 +638,14 @@ def main():
     ap.add_argument("--no-stock-cuda", action="store_true", help="skip the stock torch CUDA baseline legs")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size parity check against fp32 ATen")
     ap.add_argument("--no-defer", action="store_true", help="weight-gradient GEMMs on the compute stream (no side stream)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, parameters, running statistics and gradients of the "
+                         "last device-resident timed step to DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path's timed steps; --impl reference has none")
     if args.impl == "reference":
         run_reference(args)
     else:

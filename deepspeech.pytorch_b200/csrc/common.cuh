@@ -117,7 +117,8 @@ __device__ __forceinline__ double warp_sum_d(double v) {
 // ---- internal cross-file entry points -------------------------------------------------------
 // C[M,N] = alpha*op(A)op(B) + beta*C (row-major, fp32 FFMA kernel; any shape/stride)
 int gemm_simt(int transA, int transB, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
-              int ldb, float beta, float* C, int ldc, cudaStream_t st);
+              int ldb, float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st);
+size_t gemm_simt_workspace_bytes(int M, int N, int K);
 // tcgen05 TF32 kernel.  Returns 1 if the shape is not eligible (caller falls back to gemm_simt).
 int gemm_tc(int transA, int transB, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
             int ldb, float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st);

@@ -276,11 +276,12 @@ __global__ void bn_bwd_reduce_kernel(int B, int D, int T, const float* __restric
 }
 
 // Backward pass 2:  dz = 1[t<len] * gamma*invstd*(du - S1/N - zhat*S2/N)  in place over du,
-// plus db[c] += sum dz (bias gradient of the producing convolution).
+// plus the block's share of db[c] = sum dz (bias gradient of the producing convolution) in db_part[c][b][block],
+// summed by bias_grad_kernel in a fixed order.
 __global__ void bn_bwd_apply_kernel(int B, int D, int T, double inv_count, const float* __restrict__ z,
                                     const float* __restrict__ mi, const float* __restrict__ gamma,
                                     const int32_t* __restrict__ len, const double* __restrict__ sums,
-                                    float* __restrict__ du_dz, float* __restrict__ dbias) {
+                                    float* __restrict__ du_dz, float* __restrict__ db_part) {
   // grid (ceil(T*D/256), CO, B)
   const int c = blockIdx.y, b = blockIdx.z;
   const size_t base = ((size_t)b * CO + c) * D * T;
@@ -303,8 +304,23 @@ __global__ void bn_bwd_apply_kernel(int B, int D, int T, double inv_count, const
   if (threadIdx.x == 0) {
     float tot = 0.f;
     for (int w = 0; w < (int)blockDim.x / 32; ++w) tot += red[w];
-    atomicAdd(&dbias[c], tot);
+    db_part[((size_t)c * gridDim.z + b) * gridDim.x + blockIdx.x] = tot;
   }
+}
+
+// dbias[c] = sum of the n partials of channel c; grid CO, block 256; fixed summation order
+__global__ void bias_grad_kernel(int n, const float* __restrict__ db_part, float* __restrict__ dbias) {
+  __shared__ float red[256];
+  const float* src = db_part + (size_t)blockIdx.x * n;
+  float acc = 0.f;
+  for (int i = threadIdx.x; i < n; i += 256) acc += src[i];
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) dbias[blockIdx.x] = red[0];
 }
 
 __global__ void bn_bwd_params2d_kernel(const double* __restrict__ sums, float* __restrict__ dgamma,
@@ -448,13 +464,18 @@ int conv_tc_run(const float* in_cl, int B, int T, int R_in, int R_out, const flo
                 double* stat_sums, cudaStream_t st);
 int nchw_to_cl(int B, int R, int T, const float* in, float* out, cudaStream_t st);
 int pack_conv2_tc(const float* w2, float* wn_fwd, float* wd_bwd, cudaStream_t st);
-int conv2_wgrad_tc(const float* dz2, const float* a1, float* a1_shifted, int B, int T, float* dw2, cudaStream_t st);
-int conv1_wgrad_tc(const float* dz1, const float* x, float* xs, int B, int T, int Tp, float* dw1, cudaStream_t st);
+int conv2_wgrad_tc(const float* dz2, const float* a1, float* a1_shifted, int B, int T, float* dw2, float* part,
+                   cudaStream_t st);
+int conv1_wgrad_tc(const float* dz1, const float* x, float* xs, int B, int T, int Tp, float* dw1, float* part,
+                   cudaStream_t st);
+size_t conv_wgrad_tc_part_floats();
 
 struct ConvWs {
   float *wpk1, *wpk2, *wTe, *wTo, *du2, *da1;
   float *taps_f, *taps_b, *cl;     // tensor-core path: packed taps (21x352x32 each), channels-last staging
   float* shifted;                  // tensor-core weight gradient: a1 delayed by 0,1,2,3 time steps
+  float* wpart;                    // tensor-core weight gradients: per-CTA partial sums
+  float* dbpart;                   // conv bias gradients: per-block partial sums (CO x B x blocks)
   double* sums;   // 4 x 64 doubles: fwd stats 1, fwd stats 2, bwd sums 2, bwd sums 1
 };
 static size_t conv_ws_carve(int B, int T, void* base, ConvWs* w) {
@@ -473,6 +494,8 @@ static size_t conv_ws_carve(int B, int T, void* base, ConvWs* w) {
   p = (float*)take((size_t)21 * 352 * 32 * 4); if (w) w->taps_b = p;
   p = (float*)take((size_t)B * CO * DS2_CONV1_D * Tp * 4); if (w) w->cl = p;
   p = (float*)take((size_t)4 * B * CO * DS2_CONV1_D * (Tp + 4) * 4); if (w) w->shifted = p;
+  p = (float*)take(conv_wgrad_tc_part_floats() * 4); if (w) w->wpart = p;
+  p = (float*)take((size_t)CO * B * cdiv((long long)DS2_CONV1_D * Tp, 256) * 4); if (w) w->dbpart = p;
   return off;
 }
 
@@ -543,8 +566,6 @@ int ds2_conv_frontend_bwd(int B, int T, const float* x, const int32_t* out_len, 
   double* s1 = W.sums + 192;
   DS2_PROF("conv_bwd", st);
   DS2_CHECK_CUDA(cudaMemsetAsync(s2, 0, 128 * sizeof(double), st));
-  DS2_CHECK_CUDA(cudaMemsetAsync(db2, 0, CO * sizeof(float), st));
-  DS2_CHECK_CUDA(cudaMemsetAsync(db1, 0, CO * sizeof(float), st));
   DS2_CHECK_CUDA(cudaMemsetAsync(dw2, 0, sizeof(float) * CO * CO * 21 * 11, st));
   DS2_CHECK_CUDA(cudaMemsetAsync(dw1, 0, sizeof(float) * CO * 41 * 11, st));
 
@@ -553,7 +574,8 @@ int ds2_conv_frontend_bwd(int B, int T, const float* x, const int32_t* out_len, 
              stats + 64, g2, be2, out_len, dy, W.du2, s2);
   DS2_LAUNCH(bn_bwd_params2d_kernel, 1, 32, 0, st, s2, dg2, dbe2);
   DS2_LAUNCH(bn_bwd_apply_kernel, dim3(cdiv(D2 * Tp, 256), CO, B), 256, 0, st, B, D2, Tp, 1.0 / ((double)B * D2 * Tp),
-             z2, stats + 64, g2, out_len, s2, W.du2, db2);
+             z2, stats + 64, g2, out_len, s2, W.du2, W.dbpart);
+  DS2_LAUNCH(bias_grad_kernel, CO, 256, 0, st, B * cdiv(D2 * Tp, 256), W.dbpart, db2);
   // ---- conv2 gradients.  Nobody needs dW2 before the optimizer: with a side stream set the weight gradient runs there,
   // next to the data gradient and the (elementwise, HBM-bound) BN1 backward of the main stream, and is joined before
   // the conv1 weight gradient reuses its staging buffer.
@@ -569,7 +591,7 @@ int ds2_conv_frontend_bwd(int B, int T, const float* x, const int32_t* out_len, 
         wst = side;
         forked = true;
       }
-      wrc = conv2_wgrad_tc(W.du2, a1, W.shifted, B, Tp, dw2, wst);
+      wrc = conv2_wgrad_tc(W.du2, a1, W.shifted, B, Tp, dw2, W.wpart, wst);
       if (wrc < 0) return wrc;
       if (forked) {
         int mrc = side_mark_workspace(ws, side);
@@ -608,7 +630,8 @@ int ds2_conv_frontend_bwd(int B, int T, const float* x, const int32_t* out_len, 
              z1, stats, g1, be1, out_len, W.da1, W.da1, s1);
   DS2_LAUNCH(bn_bwd_params2d_kernel, 1, 32, 0, st, s1, dg1, dbe1);
   DS2_LAUNCH(bn_bwd_apply_kernel, dim3(cdiv(D1 * Tp, 256), CO, B), 256, 0, st, B, D1, Tp, 1.0 / ((double)B * D1 * Tp),
-             z1, stats, g1, out_len, s1, W.da1, db1);
+             z1, stats, g1, out_len, s1, W.da1, W.dbpart);
+  DS2_LAUNCH(bias_grad_kernel, CO, 256, 0, st, B * cdiv(D1 * Tp, 256), W.dbpart, db1);
   if (forked) {   // dW2 done (and its staging buffer free) before this call returns
     int jrc = side_wait_for_workspace(ws, st);
     if (jrc) return jrc;
@@ -617,7 +640,7 @@ int ds2_conv_frontend_bwd(int B, int T, const float* x, const int32_t* out_len, 
     // conv1 weight gradient on tcgen05 (reuses the conv2 weight gradient's staging buffer, which is free by now)
     int wrc = 1;
     if (tensor_core_mode() && !getenv("DS2_NO_CONV_TC") && !getenv("DS2_NO_CONV1_TC_WGRAD")) {
-      wrc = conv1_wgrad_tc(W.da1, x, W.shifted, B, T, Tp, dw1, st);
+      wrc = conv1_wgrad_tc(W.da1, x, W.shifted, B, T, Tp, dw1, W.wpart, st);
       if (wrc < 0) return wrc;
     }
     if (wrc == 1) DS2_LAUNCH(conv1_dw_kernel, dim3(3, B, C1_DSPLIT), 128, 0, st, B, T, Tp, W.da1, x, dw1);

@@ -277,7 +277,7 @@ int conv_tc_run(const float* in_cl, int B, int T, int R_in, int R_out, const flo
 // GEMM over time (K = t), organised around the INPUT row r = 2d+kh-10: one fetch of the row's eleven shifted tiles
 // (B operand, N = (kw,ci) = 352) serves every vertical tap kh of r's parity, whose dz2 rows d = (r+10-kh)/2 are
 // stacked in M: a CTA owns a group of 4 taps (M = 4 x 32 co = 128) and a slice of the (b, r) pairs, accumulates them
-// all in TMEM (352 columns) and finally adds its 128 x 352 tile into dW with fp32 atomics.  Rows d outside the output
+// all in TMEM (352 columns) and finally stores its 128 x 352 tile into its slice of the partial sums (summed per slice in a fixed order).  Rows d outside the output
 // are zero-filled by TMA.  (The first version looped over (b, d) for one kh with M = 32 of 64: every input row was
 // fetched once per tap, 19 GB of L2 -> shared-memory traffic per launch = 11 TB/s, the limit; stacking the taps cuts
 // it to 7.6 GB and fills the M = 128 data path.)
@@ -303,7 +303,7 @@ struct WgradParams {
   CUtensorMap tmS2;   // same tensor, box = 2 copies
   CUtensorMap tmS1;   // same tensor, box = 1 copy
   int B, T, slices;
-  float* dw2;
+  float* part;        // slices x 32*32*21*11: each CTA stores its partial sum, summed per slice in a fixed order
 };
 // shared-memory N block j (32 ci rows each) holds tap kw = KW_OF_BLOCK[j]:
 //   box (t0-4, copies 0,1) -> kw 1,0 | (t0, copies 0..3) -> kw 5,4,3,2 | (t0+4, copies 0..3) -> kw 9,8,7,6 | (t0+8, copy 3) -> kw 10
@@ -420,7 +420,7 @@ __global__ void __launch_bounds__(wg::THREADS, 1) conv2_wgrad_tc_kernel(const __
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(blk * 32), v);
 #pragma unroll
         for (int ci = 0; ci < 32; ++ci)
-          atomicAdd(&p.dw2[(((size_t)co * 32 + ci) * KH + kh) * 11 + kw], v[ci]);
+          p.part[(size_t)blockIdx.y * (32 * 32 * KH * 11) + (((size_t)co * 32 + ci) * KH + kh) * 11 + kw] = v[ci];
       }
     }
   }
@@ -429,10 +429,21 @@ __global__ void __launch_bounds__(wg::THREADS, 1) conv2_wgrad_tc_kernel(const __
   if (warp == 1) tmem_dealloc<512>(tmem_base);
 }
 
-// dz2: (B,32,41,T) NCHW gate... conv2 output gradient; a1: (B,32,81,T) NCHW; dw2 (32,32,21,11) must be zeroed.
+// out[e] = sum_s part[s * n + e], s in increasing order: the weight gradients do not depend on which CTA finishes first
+__global__ void sum_slices_kernel(size_t n, int slices, const float* __restrict__ part, float* __restrict__ out) {
+  for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+    float acc = 0.f;
+    for (int s = 0; s < slices; ++s) acc += part[(size_t)s * n + e];
+    out[e] = acc;
+  }
+}
+
+constexpr int WGRAD_SLICES = 24;
+// dz2: (B,32,41,T) NCHW gate... conv2 output gradient; a1: (B,32,81,T) NCHW; dw2 (32,32,21,11) is overwritten;
+// part: conv_wgrad_tc_part_floats() floats.
 // Returns 1 when the shape is not eligible (row pitch T*4 bytes must be a multiple of 16).
 int conv2_wgrad_tc(const float* dz2, const float* a1, float* a1_shifted /* 4*B*32*81*(T+4) floats */, int B, int T,
-                   float* dw2, cudaStream_t st) {
+                   float* dw2, float* part, cudaStream_t st) {
   if (T % 4 != 0) return 1;
   WgradParams p{};
   {
@@ -458,13 +469,16 @@ int conv2_wgrad_tc(const float* dz2, const float* a1, float* a1_shifted /* 4*B*3
     int rc = make_tmap_4d_f32(&p.tmDz, dz2, dims, str, box);
     if (rc) return rc;
   }
-  p.B = B; p.T = T; p.slices = 24; p.dw2 = dw2;   // 2 parities x 3 tap groups x 24 slices = 144 CTAs
+  p.B = B; p.T = T; p.slices = WGRAD_SLICES; p.part = part;   // 2 parities x 3 tap groups x 24 slices = 144 CTAs
+  const size_t n = (size_t)32 * 32 * 21 * 11;
+  DS2_CHECK_CUDA(cudaMemsetAsync(part, 0, sizeof(float) * n * p.slices, st));
   static DeviceOnce attr_once;
   if (attr_once.first()) {
     DS2_CHECK_CUDA(cudaFuncSetAttribute(conv2_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg::SMEM_BYTES));
     attr_once.done();
   }
   DS2_LAUNCH(conv2_wgrad_tc_kernel, dim3(2 * wg::GROUPS, p.slices), wg::THREADS, wg::SMEM_BYTES, st, p);
+  DS2_LAUNCH(sum_slices_kernel, cdiv((int)n, 256), 256, 0, st, n, p.slices, part, dw2);
   return DS2_OK;
 }
 
@@ -498,7 +512,7 @@ struct Wgrad1Params {
   CUtensorMap tmX8;   // 5-D (T'+4, 161, B, 2 q, 4 s), box (32, 8, 1, 2, 4)
   CUtensorMap tmX4;   // same tensor, box (32, 8, 1, 2, 2)
   int B, Tp;
-  float* dw1;
+  float* part;        // (24 slices x DI output rows) x 32*41*11, summed in a fixed order like conv2's
 };
 
 __global__ void conv1_shift_copies_kernel(int B, int T, int Tp, const float* __restrict__ x, float* __restrict__ xs) {
@@ -595,7 +609,8 @@ __global__ void __launch_bounds__(w1::THREADS, 1) conv1_wgrad_tc_kernel(const __
 #pragma unroll
       for (int c = 0; c < 32; ++c) {
         const int n = blk * 32 + c, kw = KW1_OF_GROUP[n / RJ], kh = RJ * cls + (n % RJ) - 2 * i;
-        if (kw >= 0 && kh >= 0 && kh < 41) atomicAdd(&p.dw1[((size_t)co * 41 + kh) * 11 + kw], v[c]);
+        if (kw >= 0 && kh >= 0 && kh < 41)
+          p.part[((size_t)blockIdx.y * DI + i) * (32 * 41 * 11) + ((size_t)co * 41 + kh) * 11 + kw] = v[c];
       }
     }
   }
@@ -604,9 +619,16 @@ __global__ void __launch_bounds__(w1::THREADS, 1) conv1_wgrad_tc_kernel(const __
   if (warp == 1) tmem_dealloc<128>(tmem_base);
 }
 
+size_t conv_wgrad_tc_part_floats() {
+  const size_t n2 = (size_t)32 * 32 * 21 * 11, n1 = (size_t)w1::DI * 32 * 41 * 11;
+  return (size_t)WGRAD_SLICES * (n2 > n1 ? n2 : n1);
+}
+
 // dz1: (B,32,81,T') gradient of the conv1 output (after the BN1 / Hardtanh backward); x: (B,1,161,T); dw1 (32,1,41,11)
-// must be zeroed.  xs: 8 * B * 161 * (T'+4) floats.  Returns 1 when the shape is not eligible (T' % 4 != 0).
-int conv1_wgrad_tc(const float* dz1, const float* x, float* xs, int B, int T, int Tp, float* dw1, cudaStream_t st) {
+// is overwritten.  xs: 8 * B * 161 * (T'+4) floats; part: conv_wgrad_tc_part_floats() floats.  Returns 1 when the
+// shape is not eligible (T' % 4 != 0).
+int conv1_wgrad_tc(const float* dz1, const float* x, float* xs, int B, int T, int Tp, float* dw1, float* part,
+                   cudaStream_t st) {
   if (Tp % 4 != 0) return 1;
   Wgrad1Params p{};
   const unsigned long long U = (unsigned long long)Tp + 4, F = DS2_NUM_FREQ;
@@ -629,13 +651,17 @@ int conv1_wgrad_tc(const float* dz1, const float* x, float* xs, int B, int T, in
     int rc = make_tmap_4d_f32(&p.tmDz, dz1, dims, str, box);
     if (rc) return rc;
   }
-  p.B = B; p.Tp = Tp; p.dw1 = dw1;
+  p.B = B; p.Tp = Tp; p.part = part;
+  const size_t n = (size_t)32 * 41 * 11;
+  const int slices = WGRAD_SLICES * w1::DI;
+  DS2_CHECK_CUDA(cudaMemsetAsync(part, 0, sizeof(float) * n * slices, st));
   static DeviceOnce attr_once;
   if (attr_once.first()) {
     DS2_CHECK_CUDA(cudaFuncSetAttribute(conv1_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, w1::SMEM_BYTES));
     attr_once.done();
   }
-  DS2_LAUNCH(conv1_wgrad_tc_kernel, dim3(w1::CLASSES, 24), w1::THREADS, w1::SMEM_BYTES, st, p);
+  DS2_LAUNCH(conv1_wgrad_tc_kernel, dim3(w1::CLASSES, WGRAD_SLICES), w1::THREADS, w1::SMEM_BYTES, st, p);
+  DS2_LAUNCH(sum_slices_kernel, cdiv((int)n, 256), 256, 0, st, n, slices, part, dw1);
   return DS2_OK;
 }
 

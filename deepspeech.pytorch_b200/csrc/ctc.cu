@@ -4,7 +4,7 @@
 //   kernel 2  one CTA per (utterance, sweep): the alpha sweep and the beta sweep of an utterance
 //             run CONCURRENTLY in two CTAs (they are independent), states across threads, the
 //             previous time step double-buffered in shared memory, one __syncthreads per step
-//   kernel 3  one warp per (t,b): posterior per class via shared atomics over the 2L+1 states,
+//   kernel 3  one warp per (t,b): posterior per class summed over the 2L+1 states in a fixed order,
 //             grad = softmax - posterior (fused log-softmax backward), zero for t >= in_len and for
 //             infeasible utterances (zero_infinity).
 // Integer indexing (extended target, skip rule, lengths) is exact; arithmetic fp32 like ATen.
@@ -191,12 +191,26 @@ __global__ void ctc_grad_kernel(int T, int B, int C, int Smax, const float* __re
   const int64_t* tg = targets + tgt_off[b];
   // log posterior(s) = alpha + beta - lp - ll, with the big scalars combined in double first
   const float kt = (float)(offs_a[(size_t)b * T + t] + offs_b[(size_t)b * T + t] - ll);
-  for (int s = lane; s < S; s += 32) {
-    int l = (s & 1) ? (int)tg[s >> 1] : blank;
-    float v = a[s] + be[s];
-    if (v != -CUDART_INF_F) atomicAdd(&post[l], expf(v - lpr[l] + kt));
+  // lanes with the same label (every even s is the blank; repeated labels) are summed in lane order and added by
+  // one lane per pass, so the gradient does not depend on the order in which shared-memory atomics would land
+  for (int s0 = 0; s0 < S; s0 += 32) {
+    const int s = s0 + lane;
+    int l = -1;
+    float e = 0.f;
+    if (s < S) {
+      l = (s & 1) ? (int)tg[s >> 1] : blank;
+      const float v = a[s] + be[s];
+      if (v != -CUDART_INF_F) e = expf(v - lpr[l] + kt);
+    }
+    const unsigned grp = __match_any_sync(0xffffffffu, l);
+    float tot = 0.f;
+    for (int k = 0; k < 32; ++k) {
+      const float ek = __shfl_sync(0xffffffffu, e, k);
+      if ((grp >> k) & 1u) tot += ek;
+    }
+    if (l >= 0 && lane == __ffs(grp) - 1) post[l] += tot;
+    __syncwarp();
   }
-  __syncwarp();
   for (int c = lane; c < C; c += 32) g[c] = expf(lpr[c]) - post[c];
 }
 

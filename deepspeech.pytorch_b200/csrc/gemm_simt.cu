@@ -12,8 +12,10 @@ template <bool TA, bool TB>
 __global__ void __launch_bounds__(256) gemm_simt_kernel(int M, int N, int K, float alpha,
                                                         const float* __restrict__ A, int lda,
                                                         const float* __restrict__ B, int ldb, float beta,
-                                                        float* __restrict__ C, int ldc, int k_per_split) {
-  // gridDim.z > 1: split-K, partial products are atomically added into a pre-scaled C
+                                                        float* __restrict__ C, int ldc, int k_per_split,
+                                                        float* __restrict__ part) {
+  // gridDim.z > 1: split-K, every CTA stores alpha * its partial product into part[z] (M x N), summed by
+  // splitk_reduce_kernel in a fixed order
   __shared__ __align__(16) float As[BK][BM + 4];
   __shared__ __align__(16) float Bs[BK][BN + 4];
   const int tid = threadIdx.x;
@@ -87,7 +89,7 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(int M, int N, int K, flo
       float* c = C + (size_t)gm * ldc + gn;
       float v = alpha * acc[i][j];
       if (gridDim.z > 1) {
-        atomicAdd(c, v);
+        part[((size_t)blockIdx.z * M + gm) * N + gn] = v;
       } else {
         if (beta != 0.f) v += beta * (*c);
         *c = v;
@@ -96,39 +98,63 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(int M, int N, int K, flo
   }
 }
 
-__global__ void scale_matrix_kernel(int M, int N, float beta, float* __restrict__ C, int ldc) {
-  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (size_t)M * N) return;
+// C = beta * C + sum_z part[z], z in increasing order
+__global__ void splitk_reduce_kernel(int M, int N, int splits, const float* __restrict__ part, float beta,
+                                     float* __restrict__ C, int ldc) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, n = (size_t)M * N;
+  if (i >= n) return;
+  float v = 0.f;
+  for (int z = 0; z < splits; ++z) v += part[(size_t)z * n + i];
   float* c = C + (i / N) * ldc + (i % N);
-  *c = (beta == 0.f) ? 0.f : beta * (*c);
+  *c = (beta == 0.f) ? v : fmaf(beta, *c, v);
+}
+
+// K split for long reductions onto few output tiles (weight gradients); returns the number of splits (1: none)
+static int simt_splits(int M, int N, int K, int* k_per_split) {
+  *k_per_split = K > 0 ? K : 1;
+  const int tiles = cdiv(N, BN) * cdiv(M, BM);
+  if (tiles >= 74 || K < 2048) return 1;
+  int splits = 148 / tiles;
+  if (splits > K / 256) splits = K / 256;
+  if (splits <= 1) return 1;
+  const int kps = cdiv(cdiv(K, splits), BK) * BK, gz = cdiv(K, kps);
+  if (gz > 1) *k_per_split = kps;
+  return gz > 1 ? gz : 1;
+}
+
+size_t gemm_simt_workspace_bytes(int M, int N, int K) {
+  int kps;
+  const int gz = simt_splits(M, N, K, &kps);
+  return gz > 1 ? (size_t)gz * M * N * sizeof(float) : 0;
 }
 
 int gemm_simt(int transA, int transB, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
-              int ldb, float beta, float* C, int ldc, cudaStream_t st) {
+              int ldb, float beta, float* C, int ldc, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (M <= 0 || N <= 0) return DS2_OK;
   dim3 grid(cdiv(N, BN), cdiv(M, BM));
   int k_per_split = K > 0 ? K : 1;
-  int tiles = grid.x * grid.y;
-  if (tiles < 74 && K >= 2048) {  // long reduction, few output tiles (weight gradients): split K over the SMs
-    int splits = 148 / tiles;
-    if (splits > K / 256) splits = K / 256;
-    if (splits > 1) {
-      int kps = cdiv(cdiv(K, splits), BK) * BK;
-      int gz = cdiv(K, kps);
-      if (gz > 1) {
-        k_per_split = kps;
-        grid.z = gz;
-        DS2_LAUNCH(scale_matrix_kernel, cdiv((long long)M * N, 256), 256, 0, st, M, N, beta, C, ldc);
-      }
+  float* part = nullptr;
+  {  // long reduction, few output tiles (weight gradients): split K over the SMs when the workspace holds the partials
+    int kps;
+    const int gz = simt_splits(M, N, K, &kps);
+    if (gz > 1 && ws && ws_bytes >= gemm_simt_workspace_bytes(M, N, K)) {
+      k_per_split = kps;
+      grid.z = gz;
+      part = static_cast<float*>(ws);
     }
   }
   if (transA) {
-    if (transB) DS2_LAUNCH((gemm_simt_kernel<true, true>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split);
-    else DS2_LAUNCH((gemm_simt_kernel<true, false>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split);
+    if (transB) DS2_LAUNCH((gemm_simt_kernel<true, true>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split,
+               part);
+    else DS2_LAUNCH((gemm_simt_kernel<true, false>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split,
+               part);
   } else {
-    if (transB) DS2_LAUNCH((gemm_simt_kernel<false, true>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split);
-    else DS2_LAUNCH((gemm_simt_kernel<false, false>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split);
+    if (transB) DS2_LAUNCH((gemm_simt_kernel<false, true>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split,
+               part);
+    else DS2_LAUNCH((gemm_simt_kernel<false, false>), grid, 256, 0, st, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, k_per_split,
+               part);
   }
+  if (part) DS2_LAUNCH(splitk_reduce_kernel, cdiv((long long)M * N, 256), 256, 0, st, M, N, (int)grid.z, part, beta, C, ldc);
   return DS2_OK;
 }
 
@@ -136,7 +162,8 @@ int gemm_simt(int transA, int transB, int M, int N, int K, float alpha, const fl
 
 extern "C" {
 size_t ds2_gemm_workspace_bytes(int transA, int transB, int M, int N, int K) {
-  return ds2::gemm_tc_workspace_bytes(transA, transB, M, N, K);
+  const size_t tc = ds2::gemm_tc_workspace_bytes(transA, transB, M, N, K), simt = ds2::gemm_simt_workspace_bytes(M, N, K);
+  return tc > simt ? tc : simt;
 }
 
 int ds2_gemm(int transA, int transB, int M, int N, int K, float alpha, const float* A, int lda, const float* B,
@@ -147,7 +174,7 @@ int ds2_gemm(int transA, int transB, int M, int N, int K, float alpha, const flo
     int r = ds2::gemm_tc(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, ws, ws_bytes, st);
     if (r <= 0) return r;  // 0 = done, <0 = error, 1 = shape not eligible -> FFMA kernel
   }
-  return ds2::gemm_simt(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, st);
+  return ds2::gemm_simt(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, ws, ws_bytes, st);
 }
 
 // fp16-operand GEMM of the precision-16 mode, exported for tests / the roofline bench: A16 (M,K), B16 (N,K) K-major

@@ -329,7 +329,17 @@ size_t ds2_rnn_workspace_bytes(const ds2_rnn_desc* d) {
          2 * align_up(D * d->H * TB * 2, 256) + 512;
   }
   n += rnn_sweep_tc_workspace_bytes(d->rnn_type, d->T, d->B, d->H, (int)D);
-  n += ds2_gemm_workspace_bytes(1, 0, (int)GH, d->In > d->H ? d->In : d->H, (int)TB);
+  {  // one slot shared by every ds2_gemm of the layer: the largest need among its shapes (the FFMA path keeps its
+     // split-K partials there; a narrower dW_hh splits K more ways than dW_ih)
+    const int T = d->T, B = d->B, In = d->In, H = d->H, gh = (int)GH, tb = (int)TB, kr = (T - 1) * B;
+    const int rows_x = d->rnn_type == DS2_RNN_GRU ? 2 * H : gh;
+    const size_t need[] = {ds2_gemm_workspace_bytes(0, 1, tb, gh, In), ds2_gemm_workspace_bytes(1, 0, gh, In, tb),
+                           ds2_gemm_workspace_bytes(1, 0, rows_x, H, kr), ds2_gemm_workspace_bytes(1, 0, H, H, kr),
+                           ds2_gemm_workspace_bytes(0, 0, tb, In, gh)};
+    size_t g = 0;
+    for (size_t v : need) g = v > g ? v : g;
+    n += g;
+  }
   return n + 4096;
 }
 

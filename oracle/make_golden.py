@@ -3,9 +3,10 @@
 Runs only in the dev container (needs /root/reference).  For each small configuration it builds the
 reference's own `DeepSpeech` (unmodified deepspeech_pytorch/model.py, imported through
 oracle/ref_shim.py), runs `training_step` + `loss.backward()` on seeded synthetic input and stores
-inputs, the initial state_dict, logits, loss, every parameter gradient, the post-step BatchNorm
-buffers, per-block activations (forward hooks) and an eval-mode forward (softmax + final RNN
-states).  These fixtures are what pins oracle/ds2_oracle.py and the CUDA path to the reference.
+digests of the inputs and of the initial state_dict, logits, loss, every parameter gradient, the
+post-step BatchNorm buffers, per-block activations (forward hooks) and an eval-mode forward (softmax +
+final RNN states), in the layout of oracle/golden_format.py.  These fixtures are what pins
+oracle/ds2_oracle.py and the CUDA path to the reference.
 
     python oracle/make_golden.py            # rewrites tests/golden/*.npz
 """
@@ -18,6 +19,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+import golden_format as GF  # noqa: E402
 import ref_shim  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(HERE), "tests", "golden")
@@ -50,26 +52,13 @@ def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(1)  # deterministic reductions
     for name, (rnn_type, bidir, H, layers, ctx, B, T, lens, tlens) in CASES.items():
-        torch.manual_seed(123456)  # reference train_config.py:90
+        torch.manual_seed(GF.INIT_SEED)
         model = build(ns, rnn_type, bidir, H, layers, ctx)
-        # make BN affine / running stats non-trivial so that parity exercises them
-        g = torch.Generator().manual_seed(7)
-        with torch.no_grad():
-            for k, v in model.state_dict().items():
-                if k.endswith("running_mean"):
-                    v.copy_(0.05 * torch.randn(v.shape, generator=g))
-                elif k.endswith("running_var"):
-                    v.copy_(1.0 + 0.2 * torch.rand(v.shape, generator=g))
-                elif ("batch_norm" in k or "seq_module.1" in k or "seq_module.4" in k or "module.0" in k):
-                    if k.endswith(".weight"):
-                        v.copy_(1.0 + 0.2 * torch.randn(v.shape, generator=g))
-                    elif k.endswith(".bias"):
-                        v.copy_(0.1 * torch.randn(v.shape, generator=g))
+        g = torch.Generator().manual_seed(GF.DATA_SEED)
+        GF.perturb_batchnorm(model, g)
         sd0 = {k: v.detach().clone() for k, v in model.state_dict().items()}
 
-        x = torch.randn(B, 1, 161, T, generator=g)
-        for b, l in enumerate(lens):
-            x[b, :, :, l:] = 0
+        x = GF.spectrograms(g, B, T, lens)
         pct = torch.tensor([l / float(T) for l in lens], dtype=torch.float32)
         tsz = torch.tensor(tlens, dtype=torch.int32)
         targets = torch.randint(1, 29, (sum(tlens),), generator=g, dtype=torch.int64)
@@ -110,10 +99,11 @@ def main():
         _, offsets = dec.decode(eout, eos)
         am = eout.argmax(2)
 
+        params = [[k, list(v.shape), GF.digest(v)] for k, v in sd0.items()]
         blob = {"meta": np.array(json.dumps(dict(rnn_type=rnn_type, bidirectional=bidir, hidden_size=H,
                                                   hidden_layers=layers, lookahead_context=ctx, B=B, T=T,
+                                                  lengths=lens, x=GF.digest(x), params=params,
                                                   torch=torch.__version__)))}
-        blob["x"] = x.numpy()
         blob["targets"] = targets.numpy()
         blob["input_percentages"] = pct.numpy()
         blob["target_sizes"] = tsz.numpy()
@@ -121,15 +111,13 @@ def main():
         blob["output_sizes"] = output_sizes.numpy()
         blob["logits"] = logits.numpy()
         blob["loss"] = np.array(float(loss.detach()), np.float64)
-        for k, v in sd0.items():
-            blob["p/" + k] = v.numpy()
         for k, v in grads.items():
-            blob["g/" + k] = v.numpy()
+            GF.store(blob, "g/" + k, v.numpy())
         for k, v in sd1.items():
             if "running_" in k or "num_batches" in k:
                 blob["b1/" + k] = v.numpy()
         for k, v in taps.items():
-            blob["tap/" + k] = v.numpy()
+            GF.store(blob, "tap/" + k, v.numpy())
         blob["eval_out"] = eout.numpy()
         blob["eval_argmax"] = am.numpy().astype(np.int64)
         for b in range(B):

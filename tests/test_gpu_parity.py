@@ -468,6 +468,30 @@ def test_deferred_weight_gradient_gemms_give_the_same_gradients():
     assert rel(out[True][0], out[True][1]) > 1e-2
 
 
+def test_precision_16_train_step_is_bit_repeatable():
+    """the benchmarked mode (precision 16, tensor-core front-end incl. both conv weight gradients, gradient sinks): train
+    steps from the same parameters on the same batch give bit-identical loss and gradients, so that repeated runs of a
+    training job or of the benchmark compute the same thing.  T' = 300 is eligible for the tensor-core weight gradients,
+    and T' * B = 2400 rows make the fc head's weight gradient a split-K product"""
+    from deepspeech_pytorch_b200.optim import FlatParams
+    ds.set_precision("fp16")
+    ocfg = oracle_cfg("lstm", True, 128, 3)
+    P = O.init_params(ocfg, seed=13)
+    x, targets, pct, tsz = O.synth_batch(8, 600, seed=3, lmin=5, lmax=20)
+    model = make_model("lstm", True, 128, 3, params=P).train()
+    flat = FlatParams(model, direct_grads=True)
+    runs = []
+    for _ in range(3):
+        model.load_state_dict(P)
+        loss = model.training_step((x.cuda(), targets, pct.clone(), tsz), 0)
+        loss.backward()
+        torch.cuda.synchronize()
+        runs.append((float(loss), flat.grad.clone()))
+    for loss, grad in runs[1:]:
+        assert loss == runs[0][0]
+        assert torch.equal(grad, runs[0][1]), float((grad - runs[0][1]).abs().max())
+
+
 @pytest.mark.parametrize("cfg", ["1", "2", "3"])
 def test_gemm_f16_tile_configurations_vs_fp64(cfg, monkeypatch):
     """the precision-16 mode's GEMM (fp16 K-major operands, fp32 accumulation) in every tile configuration, incl. the
